@@ -2,6 +2,7 @@
 """Headline benchmark: audio-seconds/sec (RTFx), whisper-large-v3, 30 s windows at batch 64.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--model large-v3] [--batch 64]
+                    [--dump-outputs DIR]
 
 One *step* = one pass of the ASR hot path over one batch of synthetic speech-shaped 30 s windows:
 fused log-mel -> Whisper encoder -> cross-K/V projection -> greedy decode with the logit filters
@@ -30,6 +31,7 @@ import torch
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it (it may be read-only)
 
 METRIC = "audio-seconds/sec (RTFx) whisper-large-v3 30s@b64"
 WINDOW_S = 30.0
@@ -205,7 +207,7 @@ def run_ours(args):
         torch.cuda.synchronize()
 
     def timed(fn, steps, profile=False):
-        times, extra = [], []
+        times, extra, res = [], [], None
         for _ in range(steps):
             l2_flush.fill_(1)  # flush L2 between timed iterations (inputs are also larger than L2)
             barrier()
@@ -225,7 +227,7 @@ def run_ours(args):
                 lib.wjb_profile_read(ms, cnt, 3)
                 lib.wjb_profile_enable(0)
                 extra.append({"ms": list(ms), "launches": list(cnt), "steps_run": m.stats["decode_steps"] - s0["decode_steps"], "res": res})
-        return times, extra
+        return times, extra, res
 
     for _ in range(args.warmup):
         step_resident()
@@ -254,11 +256,13 @@ def run_ours(args):
         stage["decode"].append(ev[2].elapsed_time(ev[3]))
         return res
 
-    times, extra = timed(step_resident_staged, args.steps, profile=True)
+    times, extra, last_res = timed(step_resident_staged, args.steps, profile=True)
     for _ in range(min(args.warmup, 1)):
         step_e2e()
-    e2e_times, _ = timed(step_e2e, args.steps)
+    e2e_times, _, last_e2e = timed(step_e2e, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(Path(args.dump_outputs), last_res, last_e2e)
 
     def max_over_ranks(x):
         t = torch.tensor([x], dtype=torch.float64, device="cuda")
@@ -354,6 +358,37 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+def _padded(seqs) -> np.ndarray:
+    """Ragged token lists -> [n, longest] float64, -1 past each list's end (token ids are exact in float64)."""
+    a = np.full((len(seqs), max((len(s) for s in seqs), default=0)), -1.0)
+    for i, s in enumerate(seqs):
+        a[i, : len(s)] = s
+    return a
+
+
+def dump_outputs(out_dir: Path, res, e2e) -> None:
+    """Write what the last timed step of each arm returned to its caller as ``<name>.npy`` (float64): the resident arm's
+    per-window decode results and the e2e arm's segments, one row per segment in clip order.  Audio and weights are seeded
+    and the decode is deterministic, so two builds run with the same arguments can be compared file by file."""
+    segs = [(i, s) for i, o in enumerate(e2e) for s in o["segments"]]
+    words = [(k, w) for k, (_, s) in enumerate(segs) for w in s.get("words", [])]
+    arrays = {
+        "resident_tokens": _padded([r.tokens for r in res]),
+        "resident_avg_logprob": np.array([r.avg_logprob for r in res]),
+        "resident_sum_logprob": np.array([r.sum_logprob for r in res]),
+        "resident_no_speech_prob": np.array([r.no_speech_prob for r in res]),
+        "e2e_segment_clip": np.array([i for i, _ in segs], dtype=np.float64),
+        "e2e_tokens": _padded([s["tokens"] for _, s in segs]),
+    }
+    for key in ("seek", "start", "end", "avg_logprob", "no_speech_prob", "compression_ratio", "temperature"):
+        arrays["e2e_segment_" + key] = np.array([s[key] for _, s in segs], dtype=np.float64)
+    if words:  # --word-timestamps: [segment row, start, end, probability] per word
+        arrays["e2e_words"] = np.array([[k, w["start"], w["end"], w["probability"]] for k, w in words], dtype=np.float64)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out_dir / f"{name}.npy", a)
+
+
 def parity_check(m, model_name, clips, dec_kw, sample_len=40):
     """Outside the timed region, rank 0: rows 0-1 of the benchmarked batch (same clips, same weights, same decode options)
     against the CPU oracle -- mel, encoder hidden states, then every decode step's logits and token (oracle/parity.py)."""
@@ -384,13 +419,14 @@ def _cpu_window(model_name, sample_len, pw=None, dims=None, seed_audio=2000):
     from oracle import whisper_oracle as wo
     from whisperjav_b200.synth import speech_shaped_audio
     a = speech_shaped_audio(WINDOW_S, seed_audio)
-    t0 = time.time()
-    mel = wo.pad_or_trim(wo.log_mel_spectrogram(a, dims.n_mels, padding=wo.N_SAMPLES)[:, : len(a) // 160], wo.N_FRAMES)
-    xa = wo.encoder_forward(pw, dims, mel[None], True)
-    t1 = time.time()
-    res = wo.decode(pw, dims, None, wo.DecodingOptions(language="ja", without_timestamps=True, sample_len=sample_len,
-                                                          suppress_tokens=[-1] + list(range(dims.n_vocab - 1501, dims.n_vocab))), True, audio_features=xa)
-    t2 = time.time()
+    with wo.accumulation(torch.float32):  # the reference's arithmetic: fp32 sums (the oracle's exact float64 sums are for checking)
+        t0 = time.time()
+        mel = wo.pad_or_trim(wo.log_mel_spectrogram(a, dims.n_mels, padding=wo.N_SAMPLES)[:, : len(a) // 160], wo.N_FRAMES)
+        xa = wo.encoder_forward(pw, dims, mel[None], True)
+        t1 = time.time()
+        res = wo.decode(pw, dims, None, wo.DecodingOptions(language="ja", without_timestamps=True, sample_len=sample_len,
+                                                              suppress_tokens=[-1] + list(range(dims.n_vocab - 1501, dims.n_vocab))), True, audio_features=xa)
+        t2 = time.time()
     return t1 - t0, t2 - t1, len(res[0].tokens)
 
 
@@ -618,7 +654,13 @@ def main():
     ap.add_argument("--stream-minutes", type=float, default=120.0)
     ap.add_argument("--decode", default=None, choices=["preset", "greedy"], help="default: greedy for --workload window, preset for streams")
     ap.add_argument("--word-timestamps", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step as DIR/<name>.npy (window workload, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "window"):
+        ap.error("--dump-outputs is implemented for --impl ours --workload window")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -12,14 +12,16 @@ Each function names the upstream file it follows (upstream is *not* vendored in
 
 ``sim_fp16=True`` reproduces the rounding points of the reference's fp16 GPU run
 (``fp16=True``: ``model.half()``; every Linear/Conv/GELU/residual output is an fp16
-tensor, LayerNorm and softmax compute in fp32 and cast back, logits are ``.float()``)
-while accumulating in fp32 -- which is what tensor cores do.  Parity of the CUDA path
-is asserted against this mode.
+tensor, LayerNorm and softmax compute in fp32 and cast back, logits are ``.float()``).
+Sums of products are taken in float64 before each rounding point (``ACC_DTYPE``), so the
+result does not depend on how many host threads share a matrix product.  Parity of the
+CUDA path is asserted against this mode.
 """
 from __future__ import annotations
 
 import math
 import zlib
+from contextlib import contextmanager
 from dataclasses import dataclass, field, replace
 from typing import Dict, List, Optional, Sequence, Tuple, Union
 
@@ -144,6 +146,34 @@ def sinusoids(length: int, channels: int, max_timescale: float = 10000.0) -> tor
     return torch.cat([torch.sin(scaled_time), torch.cos(scaled_time)], dim=1)
 
 
+# Sums of products (Linear, Conv1d, attention, logits) run in ACC_DTYPE and are then rounded where the reference rounds.  A
+# float32 BLAS sum on the host depends on how many threads share it; the last-bit differences flip fp16 roundings, and the
+# flips grow through the layers to several fp16 quanta of the logits -- as large as the device-vs-oracle differences the
+# parity checks bound.  A float64 sum is exact far below fp16 precision, so the oracle gives the same numbers whatever the
+# thread count.  LayerNorm and softmax stay in float32 as upstream computes them (one row per reduction: no thread split).
+ACC_DTYPE = torch.float64
+
+
+@contextmanager
+def accumulation(dtype: torch.dtype):
+    """Run the oracle with sums of products in ``dtype``; ``torch.float32`` is the reference's own arithmetic (what
+    bench.py's CPU baseline times)."""
+    global ACC_DTYPE
+    saved, ACC_DTYPE = ACC_DTYPE, dtype
+    try:
+        yield
+    finally:
+        ACC_DTYPE = saved
+
+
+def _mm(a: torch.Tensor, b: torch.Tensor) -> torch.Tensor:
+    return (a.to(ACC_DTYPE) @ b.to(ACC_DTYPE)).float()
+
+
+def _conv1d(x, w, b, **kw):
+    return F.conv1d(x.to(ACC_DTYPE), w.to(ACC_DTYPE), None if b is None else b.to(ACC_DTYPE), **kw).float()
+
+
 class Rounder:
     """fp16 rounding points of the reference's ``fp16=True`` run (identity when off)."""
 
@@ -189,7 +219,7 @@ def _linear(x, weights, prefix, r):
     # model.py::Linear.forward: weight/bias cast to x.dtype; fp32 accumulate, fp16 store
     w = _w(weights, prefix + ".weight", r)
     b = _w(weights, prefix + ".bias", r)
-    y = x @ w.t()
+    y = _mm(x, w.t())
     if b is not None:
         y = y + b
     return r(y)
@@ -208,7 +238,7 @@ def _attention(q, k, v, n_head, causal: bool, r, capture: Optional[list] = None)
     q = q.view(n_batch, n_ctx, n_head, d).permute(0, 2, 1, 3)
     k = k.view(n_batch, k.shape[1], n_head, d).permute(0, 2, 1, 3)
     v = v.view(n_batch, v.shape[1], n_head, d).permute(0, 2, 1, 3)
-    qk = (q @ k.transpose(-1, -2)) * (d ** -0.5)
+    qk = _mm(q, k.transpose(-1, -2)) * (d ** -0.5)
     if causal and n_ctx > 1:
         t_k = k.shape[2]
         mask = torch.full((n_ctx, t_k), float("-inf")).triu_(1 + t_k - n_ctx)
@@ -216,7 +246,7 @@ def _attention(q, k, v, n_head, causal: bool, r, capture: Optional[list] = None)
     if capture is not None:
         capture.append(r(qk).float())  # fp16 matmul output under fp16=True, then timing.py's .float()
     w = r(torch.softmax(qk.float(), dim=-1))  # non-SDPA branch: softmax(qk.float()).to(q.dtype)
-    out = w @ v
+    out = _mm(w, v)
     return r(out.permute(0, 2, 1, 3).flatten(start_dim=2))
 
 
@@ -225,8 +255,8 @@ def encoder_forward(weights: Dict[str, torch.Tensor], dims: ModelDimensions, mel
     """model.py::AudioEncoder.forward.  mel [B, n_mels, 3000] -> [B, 1500, n_state]."""
     r = Rounder(sim_fp16)
     x = r(mel.float())
-    x = _gelu(r(F.conv1d(x, _w(weights, "encoder.conv1.weight", r), _w(weights, "encoder.conv1.bias", r), padding=1)), r)
-    x = _gelu(r(F.conv1d(x, _w(weights, "encoder.conv2.weight", r), _w(weights, "encoder.conv2.bias", r), stride=2, padding=1)), r)
+    x = _gelu(r(_conv1d(x, _w(weights, "encoder.conv1.weight", r), _w(weights, "encoder.conv1.bias", r), padding=1)), r)
+    x = _gelu(r(_conv1d(x, _w(weights, "encoder.conv2.weight", r), _w(weights, "encoder.conv2.bias", r), stride=2, padding=1)), r)
     x = x.permute(0, 2, 1)
     pos = weights.get("encoder.positional_embedding")
     if pos is None:
@@ -300,7 +330,7 @@ def decoder_forward(weights, dims: ModelDimensions, tokens: torch.Tensor, xa: to
         x = r(x + _linear(h, weights, p + ".mlp.2", r))
     x = _layer_norm(x, weights, "decoder.ln", r)
     state.offset = offset + T
-    return r(x @ emb.t()).float()  # fp16 matmul output, then .float()
+    return r(_mm(x, emb.t())).float()  # fp16 matmul output, then .float()
 
 
 # ----------------------------------------------------------------------------- tokenizer.py

@@ -1,7 +1,10 @@
 """Plug-in surface contracts that need no GPU (the reference's own contract tests restated:
 tests/test_anime_whisper.py:129-288, tests/test_speech_segmentation.py:170-250)."""
+import importlib
 import inspect
+import json
 import sys
+import types
 from pathlib import Path
 
 import numpy as np
@@ -13,6 +16,8 @@ from whisperjav_b200.asr import B200WhisperASR
 from whisperjav_b200.audioio import compose_srt, read_wav_mono, write_wav_pcm16
 from whisperjav_b200.generator import B200WhisperGenerator
 from whisperjav_b200.segmenter import B200SpeechSegmenter
+
+BOUNDARY = json.loads((Path(__file__).parent / "golden" / "reference_boundary_kats.json").read_text())
 
 
 def test_generator_protocol_surface():
@@ -71,38 +76,56 @@ def test_wav_and_srt_io(tmp_path):
     assert compose_srt([]) == ""
 
 
-@pytest.mark.skipif(not Path("/root/reference/whisperjav").exists(), reason="reference tree not present (GPU box)")
-def test_registration_with_reference_factories(monkeypatch):
-    import types
-    sys.path.insert(0, "/root/reference")
-    for absent in ("librosa", "soundfile"):  # imported at module level by scene_detection_backends/utils.py, not installed here
-        if absent not in sys.modules:
-            monkeypatch.setitem(sys.modules, absent, types.ModuleType(absent))
-    try:
-        done = whisperjav_b200.register()
-        assert done == {"speech_segmenter": True, "text_generator": True, "scene_detector": True}
-        from whisperjav.modules.scene_detection_backends.base import SceneDetector
-        from whisperjav.modules.scene_detection_backends.factory import SceneDetectorFactory
-        det = SceneDetectorFactory.create("b200-auditok", max_duration=20.0, pass2_max_silence_s=0.5)
-        assert isinstance(det, SceneDetector) and det.name == "b200-auditok"
-        assert det._config.max_duration == 20.0 and det._config.pass2_max_duration == 19.0 and det._config.pass2_max_silence == 0.5
-        assert SceneDetectorFactory.is_backend_available("b200-auditok") == (True, "")
-        sil = SceneDetectorFactory.create("b200-silero", silero_threshold=0.1)
-        assert isinstance(sil, SceneDetector) and sil.name == "b200-silero"
-        assert sil._silero_config.max_duration == 420.0 and sil._silero_config.brute_force_chunk_s == 29.0 and sil._silero_config.silero_threshold == 0.1
-        from whisperjav.modules.speech_segmentation import SpeechSegmenterFactory
-        from whisperjav.modules.speech_segmentation.base import SpeechSegmenter
-        from whisperjav.modules.subtitle_pipeline.generators.factory import TextGeneratorFactory
-        from whisperjav.modules.subtitle_pipeline.protocols import TextGenerator
-        seg = SpeechSegmenterFactory.create("b200-vad", config={"threshold": 0.4, "chunk_threshold_s": 2.5})
-        assert isinstance(seg, SpeechSegmenter) and seg.chunk_threshold_s == 2.5
-        ws = SpeechSegmenterFactory.create("b200-whisperseg", config={"threshold": 0.35, "max_group_duration_s": 6.0})
-        assert isinstance(ws, SpeechSegmenter) and ws.name == "b200-whisperseg" and ws.max_speech_duration_s == 6.0
-        gen = TextGeneratorFactory.create("b200-whisper", model_id="tiny", device="cuda", dtype="float16",
-                                          no_repeat_ngram_size=0, max_new_tokens=444)
-        assert isinstance(gen, TextGenerator)
-    finally:
-        sys.path.remove("/root/reference")
+@pytest.fixture()
+def reference_registries(monkeypatch):
+    """Empty stand-ins for WhisperJAV's factory modules, at the module paths and with the dict names the reference has
+    (tests/golden/make_boundary_kats.py), so that ``register()`` runs as inside WhisperJAV without WhisperJAV installed."""
+    mods = {}
+    for mod_name, attrs in BOUNDARY["registries"].items():
+        parts = mod_name.split(".")
+        for i in range(1, len(parts) + 1):
+            name = ".".join(parts[:i])
+            if name not in mods:
+                mods[name] = types.ModuleType(name)
+                if i > 1:
+                    setattr(mods[".".join(parts[: i - 1])], parts[i - 1], mods[name])
+        for a in attrs:
+            setattr(mods[mod_name], a, {})
+    for name, m in mods.items():
+        monkeypatch.setitem(sys.modules, name, m)
+    return {n: mods[n] for n in BOUNDARY["registries"]}
+
+
+def test_registration_with_reference_factories(reference_registries):
+    """``register()`` fills the registries the reference's factories read, and every B200 class, built from its registered
+    dotted path with the keywords the reference's factory handed it, has the members of the protocol that factory promises
+    (``runtime_checkable`` protocols: isinstance checks exactly these names)."""
+    done = whisperjav_b200.register()
+    assert done == {"speech_segmenter": True, "text_generator": True, "scene_detector": True}
+    paths = {}
+    for mod_name, attrs in BOUNDARY["registries"].items():
+        for a, entries in attrs.items():
+            assert getattr(reference_registries[mod_name], a) == entries, (mod_name, a)
+            if a.endswith("REGISTRY"):
+                paths.update(entries)
+    objs = {}
+    for backend, c in BOUNDARY["factory_creations"].items():
+        module_name, class_name = paths[backend].rsplit(".", 1)   # the factories import the module and take the class by name
+        cls = getattr(importlib.import_module(module_name), class_name)
+        assert cls.__name__ == c["class"]
+        objs[backend] = obj = cls(**c["kwargs"])
+        assert [m for m in BOUNDARY["protocol_members"][c["protocol"]] if not hasattr(obj, m)] == [], backend
+    det = objs["b200-auditok"]
+    assert det.name == "b200-auditok"
+    assert det._config.max_duration == 20.0 and det._config.pass2_max_duration == 19.0 and det._config.pass2_max_silence == 0.5
+    # what the reference's SceneDetectorFactory.is_backend_available said of the dependency entries compared above
+    assert BOUNDARY["backend_available"] == {"b200-auditok": [True, ""], "b200-silero": [True, ""]}
+    sil = objs["b200-silero"]
+    assert sil.name == "b200-silero"
+    assert sil._silero_config.max_duration == 420.0 and sil._silero_config.brute_force_chunk_s == 29.0 and sil._silero_config.silero_threshold == 0.1
+    assert objs["b200-vad"].chunk_threshold_s == 2.5
+    ws = objs["b200-whisperseg"]
+    assert ws.name == "b200-whisperseg" and ws.max_speech_duration_s == 6.0
 
 
 def test_whisperseg_surface_and_postprocess_match_reference_defaults():
@@ -123,41 +146,39 @@ def test_whisperseg_surface_and_postprocess_match_reference_defaults():
     assert B200WhisperSegSegmenter(chunk_threshold_s=None, chunk_threshold=2.0).chunk_threshold_s == 2.0
 
 
-@pytest.mark.skipif(not Path("/root/reference/whisperjav").exists(), reason="reference tree not present (GPU box)")
 def test_reference_vad_grouped_framer_drives_the_b200_segmenters(monkeypatch):
-    """The reference's own VadGroupedFramer (subtitle_pipeline/framers/vad_grouped.py:77-164) run with both B200 segmenters:
-    factory -> segment() -> groups -> TemporalFrames.  The device stage is replaced by scripted probabilities (no GPU here); the
-    frames must be exactly the groups of the reference's own state machines on those probabilities."""
-    sys.path.insert(0, "/root/reference")
-    try:
-        whisperjav_b200.register()
-        from whisperjav.modules.subtitle_pipeline.framers.vad_grouped import VadGroupedFramer
-        from whisperjav_b200.segmenter import B200SpeechSegmenter
-        from whisperjav_b200.whisperseg import B200WhisperSegSegmenter
-        audio = np.zeros(480000, np.float32)
+    """The reference's own VadGroupedFramer (subtitle_pipeline/framers/vad_grouped.py:77-164) run with both B200 segmenters
+    (tests/golden/make_boundary_kats.py): factory -> segment() -> groups -> TemporalFrames.  The framer builds each segmenter with
+    the recorded keywords and calls segment() as recorded; every group becomes one frame, from its first segment's start to its
+    last segment's end, with the group's segments as that frame's speech regions.  The device stage is replaced by the scripted
+    probabilities of the reference run (no GPU here); the frames must be exactly the ones the reference's framer produced."""
+    from whisperjav_b200.whisperseg import B200WhisperSegSegmenter
 
-        class FakeVad:
-            device = "cpu"
+    class FakeVad:
+        device = "cpu"
 
-            def probs(self, a, ns):
-                import torch
-                p = torch.zeros(a.shape[0], (a.shape[1] + 511) // 512)
-                p[:, 100:200] = 0.9
-                p[:, 400:500] = 0.9
-                return p
-        monkeypatch.setattr(B200SpeechSegmenter, "_ensure_model", lambda self: FakeVad())
-        fr = VadGroupedFramer(segmenter_backend="b200-vad", max_group_duration_s=6.0, chunk_threshold_s=2.5).frame(audio, 16000)
-        assert fr.metadata["segmenter_backend"] == "b200-vad" and fr.metadata["total_segments"] == 2
-        assert [(round(f.start, 3), round(f.end, 3)) for f in fr.frames] == [(2.5, 7.7), (12.1, 17.3)]
+        def probs(self, a, ns):
+            import torch
+            p = torch.zeros(a.shape[0], (a.shape[1] + 511) // 512)
+            p[:, 100:200] = 0.9
+            p[:, 400:500] = 0.9
+            return p
 
-        def fake_probs(self, clips):
-            p = np.zeros(1500, np.float32)
-            p[100:200] = 0.9
-            return [p for _ in clips]
-        monkeypatch.setattr(B200WhisperSegSegmenter, "frame_probs", fake_probs)
-        fr = VadGroupedFramer(segmenter_backend="b200-whisperseg").frame(audio, 16000)
-        assert fr.metadata["segmenter_backend"] == "b200-whisperseg"
-        assert [(round(f.start, 3), round(f.end, 3)) for f in fr.frames] == [(1.7, 4.3)]     # SURVEY 8c: 2.0 - 0.3 .. 4.0 + 0.3
-        assert fr.metadata["speech_regions"] == [[(1.7, 4.3)]]
-    finally:
-        sys.path.remove("/root/reference")
+    def fake_probs(self, clips):
+        p = np.zeros(1500, np.float32)
+        p[100:200] = 0.9
+        return [p for _ in clips]
+    monkeypatch.setattr(B200SpeechSegmenter, "_ensure_model", lambda self: FakeVad())
+    monkeypatch.setattr(B200WhisperSegSegmenter, "frame_probs", fake_probs)
+    classes = {c.__name__: c for c in (B200SpeechSegmenter, B200WhisperSegSegmenter)}
+    assert [c["backend"] for c in BOUNDARY["framer"]] == ["b200-vad", "b200-whisperseg"]
+    for case in BOUNDARY["framer"]:
+        seg = classes[case["segmenter"]["class"]](**case["segmenter"]["kwargs"])
+        call = case["segment_call"]
+        r = seg.segment(np.zeros(call["n_samples"], np.float32), *call["args"], **call["kwargs"])
+        md = case["metadata"]
+        assert (r.method, r.num_segments, r.num_groups) == (md["segmenter_backend"], md["total_segments"], md["total_groups"])
+        groups = [g for g in r.groups if g]
+        assert md["groups_skipped"] == 0 and md["frame_count"] == len(groups)   # no group below the framer's minimum length
+        assert [[g[0].start_sec, g[-1].end_sec] for g in groups] == case["frames"], case["backend"]
+        assert [[[x.start_sec, x.end_sec] for x in g] for g in groups] == md["speech_regions"], case["backend"]
